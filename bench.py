@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the matching hot path: image-pairs/sec @640x480, indoor_ds dual-softmax (BASELINE.json).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--no-extra]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--no-extra] [--dump-outputs DIR]
 
 One "step" = one `matcher(batch)` call on a batch of 8 synthetic 640x480 grayscale pairs per GPU
 (BASELINE.json configs[1]; weak scaling: every rank processes its own 8 pairs, then ONE NCCL all-gather of the
@@ -20,6 +20,8 @@ Prints ONE JSON line (rank 0).  Keys follow the driver's contract:
   extra_workloads  the other BASELINE.json configs, same timing rules (N = 1: configs[2] shard, configs[3] sweep,
              configs[4] Sinkhorn, thr 0.2; N > 1: configs[2] = 4 pairs 832x832 per GPU + the all-gather)
 `--impl reference` times that CPU port as the whole arm (rank 0 only).
+`--dump-outputs DIR` writes the match lists of the last timed step (rank 0; the gathered lists when N > 1) as
+DIR/<key>.npy, so that two builds can be compared output for output on the same seeded inputs.
 """
 from __future__ import annotations
 
@@ -54,7 +56,14 @@ def parse():
     ap.add_argument("--no-extra", action="store_true", help="skip the extra_workloads block")
     ap.add_argument("--backbone", default="b200", choices=["b200", "torch"],
                     help="b200: implicit-GEMM convolutions on tcgen05 (default); torch: PyTorch/cuDNN fp32 backbone")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<key>.npy (float32 / float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
+    return args
 
 
 def peaks():
@@ -64,6 +73,26 @@ def peaks():
         return {"hbm_gbs": d["hbm_gbs"], "bf16_tflops": d["bf16_tflops"],
                 "bf16_tflops_sustained": d.get("bf16_tflops_sustained", d["bf16_tflops"]), "source": "measured"}
     return {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0, "source": "fallback"}
+
+
+def dump_outputs(out, dirname, max_bytes=64 << 20):
+    """Every tensor of `out` -> <dirname>/<key>.npy: floating point stays float32 / float64, integer ids become float64
+    (exact below 2^53), masks float32.  Above `max_bytes` in all, every array keeps the same seeded sample of rows."""
+    import numpy as np
+    import torch
+    arrs = {}
+    for k, v in out.items():
+        if torch.is_tensor(v):
+            a = v.detach().cpu().numpy()
+            arrs[k] = a.astype(np.float64 if a.dtype == np.float64 or np.issubdtype(a.dtype, np.integer) else np.float32)
+    total = sum(a.nbytes for a in arrs.values())
+    if total > max_bytes:
+        for k, a in arrs.items():
+            n = a.shape[0]
+            arrs[k] = a[np.sort(np.random.default_rng(0).choice(n, int(n * max_bytes / total), replace=False))]
+    os.makedirs(dirname, exist_ok=True)
+    for k, a in arrs.items():
+        np.save(os.path.join(dirname, k + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------ CPU arm
@@ -107,7 +136,7 @@ def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps, warmup = max(1, args.steps), max(0, args.warmup)
+    steps, warmup = args.steps, max(0, args.warmup)
     v, cores, m, s_per_step = cpu_pairs_per_sec(args.thr, steps, warmup)
     sample = f"{steps} timed steps of 1 pair 640x480 (of the batch of {args.batch}), M={m} matches/pair"
     line = {
@@ -320,7 +349,7 @@ def run_b200(args):
                     "achieved_tflops": flops / (avg * 1e-3) * 1e-12,
                     "frac": flops / (avg * 1e-3) * 1e-12 / pk["bf16_tflops_sustained"]}, rec, nprof
 
-    K, Wm = max(1, args.steps), max(3, args.warmup)
+    K, Wm = args.steps, max(3, args.warmup)
     main = Workload("indoor_ds", args.thr, B, H, W_IMG)
     hc, wc = H // 8, W_IMG // 8
 
@@ -411,8 +440,14 @@ def run_b200(args):
     # ---- device-resident throughput
     barrier()
     launches0 = lib.lb_launch_count()
+    last_step = None
+
+    def timed_step():
+        nonlocal last_step
+        last_step = main.step()
+
     with clk:
-        ms_steps = timed(lambda: main.step(), K)
+        ms_steps = timed(timed_step, K)
         barrier()
     launches = lib.lb_launch_count() - launches0
     my_ms = sum(ms_steps) / K
@@ -505,6 +540,11 @@ def run_b200(args):
         cpu = {"value": v, "unit": "pairs/s", "cores": cores, "kind": "port",
                "sample": f"3 timed forwards of 1 pair 640x480 after 1 warm-up ({s:.2f} s each, M={m_cpu}); "
                          "PyTorch-CPU backbone + numpy oracle of the reference hot path"}
+
+    if rank == 0 and args.dump_outputs:
+        local_out, gathered_out = last_step
+        dump_outputs(gathered_out if gathered_out is not None else
+                     {k: v for k, v in local_out.items() if k not in ("image0", "image1")}, args.dump_outputs)
 
     if rank == 0:
         line = {

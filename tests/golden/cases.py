@@ -23,7 +23,7 @@ _BASE = {
 # sizes, the historical position-encoding variant, M == 0.
 CASES = [
     {"name": "ds_thr0", "n": 2, "hw0": (96, 128), "hw1": (96, 128), "thr": 0.0, "images": "smooth",
-     "keep": ("conf", "feat_c")},
+     "keep": ("conf",)},
     {"name": "ds_thr_mid", "n": 2, "hw0": (96, 128), "hw1": (96, 128), "thr": 0.02, "images": "smooth"},
     {"name": "ds_empty", "n": 1, "hw0": (96, 128), "hw1": (96, 128), "thr": 0.97, "images": "rand"},
     {"name": "ds_masked_scaled", "n": 2, "hw0": (128, 128), "hw1": (128, 128), "thr": 0.0, "images": "smooth",

@@ -58,8 +58,6 @@ def run_case(ref, case):
     keep = case.get("keep", ())
     if "conf" in keep:
         out["conf_matrix"] = to_np(data["conf_matrix"])
-    if "feat_c" in keep:
-        out["feat_c0"], out["feat_c1"] = to_np(taps["coarse_tf"][0]), to_np(taps["coarse_tf"][1])
     # strided samples of the big taps keep every fixture small but still position-sensitive
     out["feat_c0_s"], out["feat_c1_s"] = to_np(taps["coarse_tf"][0])[:, ::7, ::5], to_np(taps["coarse_tf"][1])[:, ::7, ::5]
     nfine = 6

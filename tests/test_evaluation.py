@@ -83,7 +83,7 @@ def test_aggregation_matches_reference():
 
 def test_pair_list_loader_reads_reference_layout(tmp_path):
     """The loader understands the `assets/scannet_test_1500` layout (name [P,4] uint16, rel_pose [P,12], one 3x3
-    intrinsic per scene); when the reference checkout is present its real list is parsed as well."""
+    intrinsic per scene); the reference's real list (a copy in tests/golden/scannet_test_1500) is parsed as well."""
     from loftr_b200 import evaluation as E
     names = np.array([[707, 0, 15, 585], [708, 1, 45, 105]], np.uint16)
     rel = np.arange(24, dtype=np.float32).reshape(2, 12)
@@ -97,10 +97,9 @@ def test_pair_list_loader_reads_reference_layout(tmp_path):
     np.testing.assert_array_equal(pairs[1]["T_0to1_from_list"][:3], rel[1].reshape(3, 4))
     np.testing.assert_array_equal(pairs[1]["T_0to1_from_list"][3], [0, 0, 0, 1])
     np.testing.assert_array_equal(pairs[1]["K"], (K * 2).astype(np.float32))
-    ref = "/root/reference/assets/scannet_test_1500"
-    if os.path.isdir(ref):
-        real = E.load_scannet_pair_list(os.path.join(ref, "test.npz"), os.path.join(ref, "intrinsics.npz"))
-        assert len(real) == 1500 and real[0]["scene_id"] == "scene0707_00" and real[0]["K"].shape == (3, 3)
+    ref = os.path.join(util.GOLDEN, "scannet_test_1500")
+    real = E.load_scannet_pair_list(os.path.join(ref, "test.npz"), os.path.join(ref, "intrinsics.npz"))
+    assert len(real) == 1500 and real[0]["scene_id"] == "scene0707_00" and real[0]["K"].shape == (3, 3)
 
 
 # ------------------------------------------------------------------------------------------------ CUDA kernel

@@ -162,3 +162,29 @@ def test_bench_clock_sampler_filters_by_timestamp():
     assert s["samples"] == 1 and s["sm_mhz"] == 1700.0 and s["sampled"].startswith("within")
     c.rows = [["garbage"], row(-3.0, 1000)]
     assert c.summary()["samples"] == 0
+
+
+def test_bench_dump_outputs_dtypes_and_sampling(tmp_path):
+    """bench.py --dump-outputs: ids as float64, masks as float32, floats kept; over the byte limit every array keeps
+    the same seeded rows, so that the files of two runs stay comparable row for row."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench_under_test", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    m = 1000
+    out = {"b_ids": torch.arange(m), "gt_mask": torch.zeros(m, dtype=torch.bool), "mconf": torch.rand(m),
+           "mkpts0_f": torch.arange(2 * m, dtype=torch.float32).reshape(m, 2), "hw0_i": torch.Size([480, 640]), "bs": 8}
+    bench.dump_outputs(out, str(tmp_path / "all"))
+    got = {p.stem: np.load(p) for p in (tmp_path / "all").iterdir()}
+    assert set(got) == {"b_ids", "gt_mask", "mconf", "mkpts0_f"}
+    assert got["b_ids"].dtype == np.float64 and got["gt_mask"].dtype == np.float32
+    assert got["mconf"].dtype == np.float32 and np.array_equal(got["mconf"], out["mconf"].numpy())
+    limit = 8000
+    for d in ("s1", "s2"):
+        bench.dump_outputs(out, str(tmp_path / d), max_bytes=limit)
+    s1 = {p.stem: np.load(p) for p in (tmp_path / "s1").iterdir()}
+    s2 = {p.stem: np.load(p) for p in (tmp_path / "s2").iterdir()}
+    assert 0 < sum(a.nbytes for a in s1.values()) <= limit
+    assert all(np.array_equal(s1[k], s2[k]) for k in s1)
+    rows = s1["b_ids"].astype(np.int64)
+    assert (np.diff(rows) > 0).all() and np.array_equal(s1["mkpts0_f"], got["mkpts0_f"][rows])
