@@ -4,7 +4,8 @@
 mkdir -p gpurun_out
 cd "$(dirname "$0")/.."
 filter="${1:-.}"
-mapfile -t groups < <(python -m pytest tests/test_engine_gpu.py --collect-only -q -m gpu -p no:cacheprovider 2>/dev/null \
+mapfile -t groups < <(python -m pytest tests/test_engine_gpu.py tests/test_kernel_edges_gpu.py --collect-only -q -m gpu \
+  -p no:cacheprovider 2>/dev/null \
   | grep "::" | sed 's/\[.*//' | sort -u | grep -E "$filter")
 rc=0
 : > gpurun_out/gpu_tests.log

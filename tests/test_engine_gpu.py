@@ -21,25 +21,43 @@ def _t(x, dtype=None):
 
 
 # ------------------------------------------------------------------------------------------------ contraction core
+# (batches, M, N, K[, "shared_b" | "wide"]).  Edge cases: M = 1 / 127 / 129 (one M-tile: single-CTA launch; a one-row
+# second tile), N = 32 (128-column tiles), 160 (one partial 256-column tile), 288 (a 32-column second tile), K = 64 (one
+# k-block) / 1024; "shared_b": batched A against ONE B (b_batch_stride = 0); "wide": magnitudes 1e-3 .. 1e3 with random
+# signs, so the products of the `lo` planes carry real information.
+_GEMM_EDGE = [(1, m, n, k) for m in (1, 127, 129) for n in (32, 160, 288) for k in (64, 1024)]
+
+
 @pytest.mark.parametrize("shape", [(1, 128, 256, 64), (1, 300, 768, 256), (1, 1000, 128, 128), (2, 200, 512, 256),
-                                   (1, 1200, 384, 128), (1, 77, 256, 512)])
+                                   (1, 1200, 384, 128), (1, 77, 256, 512)] + _GEMM_EDGE +
+                         [(3, 129, 288, 64, "shared_b"), (4, 1, 32, 1024, "shared_b"), (2, 300, 160, 256, "shared_b"),
+                          (1, 129, 288, 1024, "wide"), (3, 127, 160, 512, "wide"), (2, 1, 288, 64, "wide")])
 def test_gemm_split_matches_fp64(shape):
     from loftr_b200 import _lib
     from loftr_b200.loftr import split_planes, _stream
-    b, m, n, k = shape
+    b, m, n, k = shape[:4]
+    kind = shape[4] if len(shape) > 4 else ""
+    nb = 1 if kind == "shared_b" else b
     rs = np.random.RandomState(0)
-    a = (rs.standard_normal((b * m, k)) * 3 + 1).astype(np.float32)
-    w = (rs.standard_normal((b * n, k)) * 3 + 1).astype(np.float32)
+    if kind == "wide":
+        a = (10.0 ** rs.uniform(-3, 3, (b * m, k)) * rs.choice([-1, 1], (b * m, k))).astype(np.float32)
+        w = (10.0 ** rs.uniform(-3, 3, (nb * n, k)) * rs.choice([-1, 1], (nb * n, k))).astype(np.float32)
+    else:
+        a = (rs.standard_normal((b * m, k)) * 3 + 1).astype(np.float32)
+        w = (rs.standard_normal((nb * n, k)) * 3 + 1).astype(np.float32)
     ta, tw = _t(a), _t(w)
     ah, al = split_planes(ta)
     wh, wl = split_planes(tw)
     out = torch.empty(b * m, n, dtype=torch.float32, device=DEV)
     lib = _lib.load()
     _lib.check(lib.lb_gemm_split(ah.data_ptr(), al.data_ptr(), k, m * k, wh.data_ptr(), wl.data_ptr(), k,
-                                 n * k if b > 1 else 0, out.data_ptr(), n, m * n, b, m, n, k, _stream()))
-    ref = np.einsum("bmk,bnk->bmn", a.reshape(b, m, k).astype(np.float64), w.reshape(b, n, k).astype(np.float64))
+                                 n * k if nb > 1 else 0, out.data_ptr(), n, m * n, b, m, n, k, _stream()))
+    ref = np.einsum("bmk,bnk->bmn", a.reshape(b, m, k).astype(np.float64),
+                    np.broadcast_to(w.reshape(nb, n, k), (b, n, k)).astype(np.float64))
     got = out.cpu().numpy().reshape(b, m, n)
-    assert np.abs(got - ref).max() / np.abs(ref).max() < 5e-6
+    err = np.abs(got - ref).max() / np.abs(ref).max()
+    util.record("gemm_split_" + "x".join(map(str, shape)), {"max_err_rel_to_max_ref": float(err)})
+    assert err < 5e-6
 
 
 # ------------------------------------------------------------------------------------------------ transformer
@@ -317,7 +335,18 @@ def test_large_batch_duplicate_pairs_agree():
 
 
 # ------------------------------------------------------------------------------------------------ backbone on tensor cores
-@pytest.mark.parametrize("shape", [(2, 96, 128), (1, 480, 640), (1, 136, 200)])
+# Branches of run_conv / launch_conv the small and ragged shapes reach.  An output map of h x w pixels has
+# ceil(h/8) * ceil(w/16) tiles of 8 x 16; one tile runs the single-CTA kernel (mode 0), two or more the CTA pair
+# (mode 2).  A lateral (layer2_outconv: Cout 256 at 1/4, layer1_outconv: Cout 196 at 1/2) stages its x2 upsample source
+# in shared memory (EpiConv<., 1, .>) only in mode 2, otherwise every thread gathers it (EpiConv<256|208, 2, true>).
+#   shape         tiles 1/2, 1/4, 1/8     modes (1/2, 1/4, 1/8)   layer2_outconv   layer1_outconv   coarse grid
+#   (2, 8, 8)     1, 1, 1                 0, 0, 0                 per-thread       per-thread       1 x 1
+#   (2, 16, 32)   1, 1, 1                 0, 0, 0                 per-thread       per-thread       2 x 4
+#   (3, 32, 64)   4, 1, 1                 2, 0, 0                 per-thread       staged           4 x 8
+#   (1, 8, 256)   8, 4, 2                 2, 2, 2                 staged           staged           1 x 32
+#   (1, 200, 40)  26, 7, 4                2, 2, 2                 staged           staged           25 x 5 (ragged tiles)
+@pytest.mark.parametrize("shape", [(2, 96, 128), (1, 480, 640), (1, 136, 200), (2, 8, 8), (2, 16, 32), (3, 32, 64),
+                                   (1, 8, 256), (1, 200, 40)])
 def test_tensor_core_backbone_matches_torch(shape):
     """lb_backbone_forward (implicit-GEMM convolutions, folded BN, fused residual / FPN upsample-add) against the
     PyTorch ResNetFPN_8_2 forward in fp32 (TF32 off) with non-trivial BatchNorm statistics."""
